@@ -177,6 +177,28 @@ def gen_local(torch, dev, rank, world, n_build, n_probe):
     return bk, bv, pk, pv
 
 
+DUMP_ROWS = 1 << 19    # rows kept from a larger output: 8 float64 arrays of 4 MiB at most (4 int64 join columns)
+
+
+def dump_outputs(out_dir, cols, order_by):
+    """--dump-outputs: write the result columns of one step (name -> 1-D int64/float64 CUDA tensor, all of one length) as
+    out_dir/<name>.npy, so that two builds can be compared output for output.  The kernels emit rows in no fixed order, so
+    rows are first sorted by cols[order_by], which is unique per output row; an output longer than DUMP_ROWS is cut to a
+    fixed, seeded sample of DUMP_ROWS rows.  float64 columns are stored as they are; an int64 column, which float64 cannot
+    hold exactly, as two exact float64 arrays <name>_hi (bits 63..32, signed) and <name>_lo (bits 31..0)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    order = torch.sort(cols[order_by], stable=True).indices
+    if order.numel() > DUMP_ROWS:
+        pick = np.sort(np.random.default_rng(0).choice(order.numel(), DUMP_ROWS, replace=False))
+        order = order[torch.from_numpy(pick).to(order.device)]
+    for name, t in cols.items():
+        v = t[order]
+        parts = {name: v} if v.dtype == torch.float64 else {name + "_hi": (v >> 32).double(), name + "_lo": (v & 0xFFFFFFFF).double()}
+        for part, a in parts.items():
+            np.save(os.path.join(out_dir, part + ".npy"), a.cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------------------
 # CPU legs (oracle): the only place bench.py touches oracle/
 # ---------------------------------------------------------------------------------------------------------
@@ -376,6 +398,7 @@ def run_gpu(args):
         return torch.stack([o_pv.sum(), (o_pv * o_pv).sum()])
 
     TRACE = [] if os.environ.get("BENCH_TRACE") else None
+    last_cols = []    # N = 1: device pointers of the latest step's output columns (valid until the next probe call)
 
     # ---- N > 1, mailbox exchange: candidates and (for --exchange auto) an untimed calibration -----------------------
     xmail = None
@@ -445,6 +468,7 @@ def run_gpu(args):
         """sync=True is the verifying pass: returns (rows, checksums)"""
         if world == 1:
             rows, cols, _ = join.probe([pk, pv], sync=sync)
+            last_cols[:] = cols
             return (rows, check_piece(cols, rows)) if sync else (None, None)
         if xmail is not None:
             return mail_step(xmail, sync)
@@ -571,6 +595,14 @@ def run_gpu(args):
                 "algorithmic_bytes_per_launch": BYTES_PER_PROBE_ROW * npb * world,
                 "nvlink": {"payload_gbs_per_direction_per_gpu": nvl, "reference_gbs": 770.0, "frac": nvl / 770.0,
                            "note": "16 B per exchanged row; reference = measured peer-copy bandwidth per direction (B200_PROFILING.md)"}}
+
+    if args.dump_outputs:
+        # the last timed step's result, still in the join's output buffers; it probed the same inputs as the verifying
+        # step, whose output row count `rows` was checked above
+        with torch.cuda.stream(stream):
+            dump_outputs(args.dump_outputs, {name: dview(p, rows) for name, p in
+                                             zip(("probe_key", "probe_payload", "build_key", "build_payload"), last_cols)}, "probe_payload")
+        stream.synchronize()
 
     # ---- side line (N = 1): the 50 % match variant of the same workload (SURVEY 8d input 2) ---------------------------
     side50 = None
@@ -914,7 +946,9 @@ def run_agg(args):
         o = _A(); o.__cuda_array_interface__ = {"shape": (m,), "typestr": dt, "data": (p, False), "version": 3}
         return torch.as_tensor(o, device=dev)
 
-    def one(verify=False):
+    kept = []    # --dump-outputs: (handle, rows, result column pointers) of the last timed step, closed once written out
+
+    def one(verify=False, keep=False):
         agg = DeviceAgg(plan)
         with torch.cuda.stream(stream):
             agg.push([keys, x])
@@ -926,7 +960,10 @@ def run_agg(args):
                 exp = torch.zeros(G, dtype=torch.float64, device=dev).scatter_add_(0, keys, x)
                 assert torch.allclose(s_, exp[gk], rtol=1e-6, atol=0)
         st = agg.stats()
-        agg.close()
+        if keep:
+            kept.append((agg, rows, cols))
+        else:
+            agg.close()
         return st
     for _ in range(max(3, args.warmup) - 1):
         one()
@@ -936,13 +973,20 @@ def run_agg(args):
     launches = 0
     with torch.cuda.stream(stream):
         e0.record(stream)
-    for _ in range(args.steps):
-        launches += one().kernel_launches
+    for i in range(args.steps):
+        launches += one(keep=bool(args.dump_outputs) and i == args.steps - 1).kernel_launches
     with torch.cuda.stream(stream):
         e1.record(stream)
     stream.synchronize()
     clocks = sampler.stop()
     ms = e0.elapsed_time(e1) / args.steps
+    if kept:
+        agg, rows, cols = kept.pop()
+        with torch.cuda.stream(stream):
+            dump_outputs(args.dump_outputs, {"group_key": view(cols[0], rows, "<i8"), "sum": view(cols[1], rows, "<f8"),
+                                             "count": view(cols[2], rows, "<i8")}, "group_key")
+        stream.synchronize()
+        agg.close()
     # e2e: host chunks through tg_agg_push / tg_agg_next (pinned host memory in, host result out)
     e2e = None
     if not args.skip_e2e:
@@ -1024,7 +1068,14 @@ def main():
     ap.add_argument("--skip-side", action="store_true", help="skip the 50 %% match side line (N = 1)")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--ncu-traffic-bytes", type=float, default=None, help="dram bytes per launch from the committed ncu capture")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output columns of the last one as DIR/<name>.npy (float64; rows in a canonical "
+                         f"order, a seeded sample of {DUMP_ROWS} rows of a larger output; GPU arm, one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl b200 and --gpus 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":
