@@ -404,6 +404,60 @@ int tg_topn(int device, int on_device, const tg_chunk* chk, const int32_t* col_t
             tg_mut_chunk* out, int64_t* nrows, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Sort                          replaces sortexec.SortExec (pkg/executor/sortexec/sort.go:43) for ORDER BY without LIMIT
+ * Every row of the child in ORDER BY order: items compared one after another with chunk.GetCompareFunc
+ * (SortExec.lessRow sort.go:804; util/chunk/compare.go:30-60): NULL before every value, DESC negates; signed / unsigned
+ * int family and YEAR as int64 / uint64 (unsigned flag), DURATION as int64, DOUBLE as Go cmp.Compare (NaN first, NaNs equal, -0 == +0),
+ * DATE / DATETIME / TIMESTAMP as the packed CoreTime word without its 4 fsp bits.  The device sort is stable (rows that
+ * tie on every item keep their input order); the reference's is not, so callers must not rely on it.
+ * 1..8 items over plain columns, 1..16 columns, every column 8 bytes (int family, YEAR, DURATION, DOUBLE, time);
+ * at most 2^32 - 1 rows (row ids are 32-bit).  The whole input and the result live in HBM: no spill.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct tg_sort tg_sort;
+typedef struct tg_sort_desc {
+  int32_t n_cols;                 /* child schema                                               */
+  int32_t n_items;
+  const int32_t* col_types; const uint32_t* col_flags;
+  const tg_sort_item* items;      /* ByItems as plain column refs (buildKeyColumns sort.go:789)  */
+  int32_t device;
+  int32_t reserved;
+  void* stream;                   /* cudaStream_t; NULL = library-owned stream                   */
+  int64_t expected_rows;          /* hint for buffer sizing (planner estimate); 0 = grow on demand */
+} tg_sort_desc;
+
+/* planner gate: 0 if this descriptor can run on the GPU; answers without a device               */
+int tg_sort_supported(const tg_sort_desc* desc);
+/* SortExec.Open (sort.go:155)                                                                   */
+int tg_sort_open(const tg_sort_desc* desc, tg_sort** out);
+/* SortExec.fetchChunks (sort.go:526): one child chunk from host memory, sel honoured; copied before returning */
+int tg_sort_push(tg_sort* s, const tg_chunk* chk);
+/* same, columns already resident in device memory (no sel; borrowed until tg_sort_finish)       */
+int tg_sort_push_dev(tg_sort* s, const tg_chunk* dev_chk);
+/* end of input: the sort itself (LSD radix sort of the ORDER BY items) and the gather of every column */
+int tg_sort_finish(tg_sort* s);
+/* SortExec.Next (sort.go:265): the next min(max_rows, out->capacity_rows) rows; *nrows == 0 means EOF */
+int tg_sort_next(tg_sort* s, tg_mut_chunk* out, int64_t max_rows, int64_t* nrows);
+/* device-resident result: row count + device pointers of the sorted columns and their null bitmaps (NULL: no NULLs);
+ * valid until close                                                                             */
+int tg_sort_result_dev(tg_sort* s, int64_t* out_rows, void** out_cols, void** out_nulls);
+
+typedef struct tg_sort_stats {
+  int64_t input_rows;
+  int64_t digit_passes;           /* 8-bit digit scatter passes run                              */
+  int64_t skipped_passes;         /* digit passes skipped: every row had the same digit          */
+  int64_t null_passes;            /* NULL-flag passes run                                        */
+  int64_t kernel_launches;
+  double sort_ms, gather_ms;      /* device time measured with CUDA events                       */
+  int64_t h2d_bytes, d2h_bytes;
+} tg_sort_stats;
+int tg_sort_get_stats(tg_sort* s, tg_sort_stats* out);
+/* SortExec.Close (sort.go:109); idempotent, may race with an in-flight call                    */
+int tg_sort_close(tg_sort* s);
+/* The order-preserving 64-bit key the sort gives one non-NULL value of a column (host evaluation of the device
+ * normalizer; tests and planners): keys compare as uint64 exactly as the values compare under ORDER BY.      */
+int tg_sort_key_host(int32_t mysql_type, uint32_t flag, int32_t desc, uint64_t raw, uint64_t* key);
+
+/* ---------------------------------------------------------------------------------------------
  * Key-hash repartition for the multi-GPU exchange (the B200 analogue of the MPP
  * ExchangeSender HashPartition, pkg/planner/core/operator/physicalop/physical_exchange_sender.go:115;
  * in-process analogue: partitionHashSplitter.split, pkg/executor/shuffle.go:450).

@@ -120,6 +120,33 @@ class TgAggStats(C.Structure):
                 ("finalize_ms", C.c_double), ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64)]
 
 
+class TgSortDesc(C.Structure):
+    _fields_ = [("n_cols", C.c_int32), ("n_items", C.c_int32),
+                ("col_types", C.POINTER(C.c_int32)), ("col_flags", C.POINTER(C.c_uint32)),
+                ("items", C.POINTER(TgSortItem)), ("device", C.c_int32), ("reserved", C.c_int32),
+                ("stream", C.c_void_p), ("expected_rows", C.c_int64)]
+
+
+class TgSortStats(C.Structure):
+    _fields_ = [("input_rows", C.c_int64), ("digit_passes", C.c_int64), ("skipped_passes", C.c_int64),
+                ("null_passes", C.c_int64), ("kernel_launches", C.c_int64), ("sort_ms", C.c_double),
+                ("gather_ms", C.c_double), ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64)]
+
+
+def sort_desc(schema, by_items, device: int = 0, expected_rows: int = 0, stream=None):
+    """tg_sort_desc for a child schema (FieldType list) and ORDER BY items [(column, desc)]; returns (desc, keep-alive)"""
+    tps = (C.c_int32 * max(len(schema), 1))(*[t.tp for t in schema])
+    fls = (C.c_uint32 * max(len(schema), 1))(*[t.flag for t in schema])
+    items = (TgSortItem * max(len(by_items), 1))(*[TgSortItem(int(c), int(bool(d))) for c, d in by_items])
+    d = TgSortDesc()
+    d.n_cols, d.n_items = len(schema), len(by_items)
+    d.col_types = C.cast(tps, C.POINTER(C.c_int32))
+    d.col_flags = C.cast(fls, C.POINTER(C.c_uint32))
+    d.items = C.cast(items, C.POINTER(TgSortItem))
+    d.device, d.stream, d.expected_rows = device, stream, expected_rows
+    return d, (tps, fls, items)
+
+
 # every symbol include/tidbgpu.h declares; tests/test_abi_exports.py checks the .so exports them all
 EXPORTED_SYMBOLS = [
     "tg_last_error", "tg_abi_version", "tg_device_count", "tg_device_info", "tg_fixed_len",
@@ -133,6 +160,8 @@ EXPORTED_SYMBOLS = [
     "tg_agg_next", "tg_agg_close", "tg_agg_result_dev", "tg_agg_get_stats",
     "tg_vec_compare_int", "tg_vec_compare_real", "tg_vec_arith_int", "tg_vec_arith_real",
     "tg_vec_filter", "tg_topn",
+    "tg_sort_supported", "tg_sort_open", "tg_sort_push", "tg_sort_push_dev", "tg_sort_finish", "tg_sort_next",
+    "tg_sort_result_dev", "tg_sort_get_stats", "tg_sort_close", "tg_sort_key_host",
     "tg_partition_by_key", "tg_partition_of_key", "tg_partition_exchange", "tg_partition_exchange_cf", "tg_partition_exchange_cf_ex", "tg_partition_exchange_cf_spill", "tg_partition_count",
     "tg_mail_signal", "tg_mail_wait", "tg_peer_copy_regions",
     "tg_ipc_export", "tg_ipc_open", "tg_ipc_close",
@@ -160,6 +189,7 @@ def load_lib() -> C.CDLL:
     lib.tg_last_error.restype = C.c_char_p
     lib.tg_partition_of_key.restype = C.c_int32
     lib.tg_partition_of_key.argtypes = [C.c_int64, C.c_int32]
+    lib.tg_sort_key_host.argtypes = [C.c_int32, C.c_uint32, C.c_int32, C.c_uint64, C.POINTER(C.c_uint64)]
     _lib = lib
     return lib
 

@@ -17,7 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "build")
 LIB = os.path.join(CSRC, "libtidbgpu.so")
-SOURCES = ["runtime.cu", "join.cu", "agg.cu", "vec.cu", "partition.cu", "codec.cu", "topn.cu"]
+SOURCES = ["runtime.cu", "join.cu", "agg.cu", "vec.cu", "partition.cu", "codec.cu", "topn.cu", "sort.cu"]
 HEADERS = ["common.cuh", "join_kernels.cuh", "partition_kernels.cuh", "tma.cuh", "agg_update.cuh", os.path.join("..", "..", "include", "tidbgpu.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "--expt-relaxed-constexpr"]

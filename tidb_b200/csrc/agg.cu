@@ -603,12 +603,6 @@ __global__ void k_agg_rehash_mk(AggTable oldt, AggTable newt, int nstates) {
 #include "agg_update.cuh"
 namespace tg {
 
-struct AggHostStage {
-  std::vector<std::unique_ptr<PinBuf>> data, nulls;
-  std::vector<char> has_nulls;
-  int64_t rows = 0;
-};
-
 }  // namespace tg
 
 using namespace tg;
@@ -651,7 +645,7 @@ struct AggImpl {
   int local_mode = -1;            // -1 undecided, 0 global atomics only, 1 CTA-local partial aggregation first
 
   // staging
-  AggHostStage stage;
+  ColumnStage stage;
   std::vector<std::unique_ptr<DevBuf>> dcols, dnulls;
 
   // result
@@ -1129,8 +1123,6 @@ static int update_device(AggImpl* a, const DevCols& cols, int64_t n) {
   return TG_OK;
 }
 
-static int64_t alogical_rows(const tg_chunk* c) { return c->sel ? c->nsel : (c->ncols > 0 ? c->cols[0].length : 0); }
-
 static int avalidate(const AggImpl* a, const tg_chunk* chk) {
   if (!chk || chk->ncols != a->ncols) return fail(TG_ERR_INVALID, "chunk column count does not match the child schema");
   int64_t phys = chk->cols[0].length;
@@ -1142,41 +1134,8 @@ static int avalidate(const AggImpl* a, const tg_chunk* chk) {
   return TG_OK;
 }
 
-static int astage_append(AggImpl* a, const tg_chunk* chk) {
-  AggHostStage& st = a->stage;
-  int64_t n = alogical_rows(chk);
-  if (n == 0) return TG_OK;
-  for (int c = 0; c < a->ncols; c++) {
-    if (!a->needed[c]) continue;
-    const tg_column& col = chk->cols[c];
-    PinBuf& d = *st.data[c];
-    TG_TRY(d.reserve((size_t)(st.rows + n) * 8));
-    uint64_t* dst = reinterpret_cast<uint64_t*>(d.p) + st.rows;
-    const uint64_t* src = reinterpret_cast<const uint64_t*>(col.data);
-    if (!chk->sel) std::memcpy(dst, src, (size_t)n * 8);
-    else for (int64_t i = 0; i < n; i++) dst[i] = src[chk->sel[i]];
-    d.used = (size_t)(st.rows + n) * 8;
-    bool bring = col.null_bitmap != nullptr;
-    if (bring || st.has_nulls[c]) {
-      PinBuf& nb = *st.nulls[c];
-      size_t need = (size_t)((st.rows + n + 7) / 8) + 1;
-      TG_TRY(nb.reserve(need));
-      if (!st.has_nulls[c]) { std::memset(nb.p, 0xff, (size_t)((st.rows + 7) / 8) + 1); st.has_nulls[c] = 1; }
-      if (bring && !chk->sel) append_bits(nb.p, st.rows, col.null_bitmap, n);
-      else for (int64_t i = 0; i < n; i++) {
-        bool nn = bring ? bit_not_null(col.null_bitmap, chk->sel ? chk->sel[i] : i) : true;
-        int64_t r = st.rows + i;
-        if (nn) nb.p[r >> 3] |= (uint8_t)(1u << (r & 7)); else nb.p[r >> 3] &= (uint8_t)~(1u << (r & 7));
-      }
-      nb.used = need;
-    }
-  }
-  st.rows += n;
-  return TG_OK;
-}
-
 static int aflush(AggImpl* a) {
-  AggHostStage& st = a->stage;
+  ColumnStage& st = a->stage;
   if (st.rows == 0) return TG_OK;
   DevCols v{};
   for (int c = 0; c < a->ncols; c++) {
@@ -1293,11 +1252,8 @@ int tg_agg_open(const tg_agg_desc* desc, tg_agg** out) {
   TG_CUDA(cudaEventCreate(&a->ev0));
   TG_CUDA(cudaEventCreate(&a->ev1));
   a->nsm = device_sm_count(a->device);
-  for (int c = 0; c < a->ncols; c++) {
-    a->stage.data.emplace_back(new PinBuf()); a->stage.nulls.emplace_back(new PinBuf());
-    a->dcols.emplace_back(new DevBuf()); a->dnulls.emplace_back(new DevBuf());
-  }
-  a->stage.has_nulls.assign(a->ncols, 0);
+  a->stage.init(a->ncols);
+  for (int c = 0; c < a->ncols; c++) { a->dcols.emplace_back(new DevBuf()); a->dnulls.emplace_back(new DevBuf()); }
   shell->impl = a.release();
   *out = shell.release();
   return TG_OK;
@@ -1307,7 +1263,7 @@ int tg_agg_push(tg_agg* h, const tg_chunk* chk) {
   TGA_LOCK(h);
   if (a->finished) return fail(TG_ERR_STATE, "push after finish");
   TG_TRY(avalidate(a, chk));
-  TG_TRY(astage_append(a, chk));
+  TG_TRY(stage_append(a->stage, chk, a->needed));
   if (a->stage.rows >= (4ll << 20)) TG_TRY(aflush(a));
   return TG_OK;
 }
@@ -1345,36 +1301,10 @@ int tg_agg_next(tg_agg* h, tg_mut_chunk* out, int64_t max_rows, int64_t* nrows) 
   int64_t lo = a->consumed;
   int64_t want = std::min<int64_t>(std::min<int64_t>(max_rows, out->capacity_rows), a->out_rows - lo);
   if (want <= 0) return TG_OK;
-  // any RequiredRows >= 1 is served: bitmaps that start inside a byte are fetched whole and shifted on the host
-  const int shift = (int)(lo & 7);
-  std::vector<std::vector<uint8_t>> shifted;
-  for (int k = 0; k < a->spec.n; k++) {
-    TG_CUDA(cudaMemcpyAsync(out->cols[k].data, a->out_cols[k]->as<uint8_t>() + (size_t)lo * 8, (size_t)want * 8, cudaMemcpyDeviceToHost, a->stream));
-    a->stats.d2h_bytes += want * 8;
-    size_t nb = (size_t)((want + 7) / 8);
-    if (a->out_bitmaps[k]->p) {
-      if (!out->cols[k].null_bitmap) return fail(TG_ERR_INVALID, "output column can be NULL but the caller passed no null bitmap");
-      if (shift == 0) TG_CUDA(cudaMemcpyAsync(out->cols[k].null_bitmap, a->out_bitmaps[k]->as<uint8_t>() + lo / 8, nb, cudaMemcpyDeviceToHost, a->stream));
-      else {
-        shifted.emplace_back((size_t)((shift + want + 7) / 8) + 1, (uint8_t)0);
-        TG_CUDA(cudaMemcpyAsync(shifted.back().data(), a->out_bitmaps[k]->as<uint8_t>() + lo / 8, shifted.back().size() - 1, cudaMemcpyDeviceToHost, a->stream));
-      }
-    } else if (out->cols[k].null_bitmap) {
-      std::memset(out->cols[k].null_bitmap, 0xff, nb);
-      if (want & 7) out->cols[k].null_bitmap[nb - 1] = (uint8_t)((1u << (want & 7)) - 1);
-    }
-  }
-  TG_CUDA(cudaStreamSynchronize(a->stream));
-  if (shift) {
-    size_t q = 0;
-    for (int k = 0; k < a->spec.n; k++) {
-      if (!a->out_bitmaps[k]->p) continue;
-      const std::vector<uint8_t>& src = shifted[q++];
-      size_t nb = (size_t)((want + 7) / 8);
-      for (size_t b = 0; b < nb; b++) out->cols[k].null_bitmap[b] = (uint8_t)((src[b] >> shift) | (src[b + 1] << (8 - shift)));
-    }
-  }
-  if (want & 7) for (int k = 0; k < a->spec.n; k++) if (a->out_bitmaps[k]->p) out->cols[k].null_bitmap[want >> 3] &= (uint8_t)((1u << (want & 7)) - 1);
+  std::vector<const void*> cols(a->spec.n);
+  std::vector<const uint8_t*> bitmaps(a->spec.n);
+  for (int k = 0; k < a->spec.n; k++) { cols[k] = a->out_cols[k]->p; bitmaps[k] = a->out_bitmaps[k]->as<uint8_t>(); }
+  TG_TRY(copy_out_rows(a->stream, a->spec.n, cols.data(), bitmaps.data(), lo, want, out, &a->stats.d2h_bytes));
   a->consumed += want;
   *nrows = want;
   return TG_OK;

@@ -9,6 +9,7 @@
 #include <vector>
 #include <mutex>
 #include <atomic>
+#include <memory>
 #include "../../include/tidbgpu.h"
 
 namespace tg {
@@ -187,6 +188,28 @@ __host__ __device__ __forceinline__ bool bit_not_null(const uint8_t* bm, int64_t
 
 // append nbits of src (starting at src bit 0) to dst at bit position pos (host side)
 void append_bits(uint8_t* dst, int64_t pos, const uint8_t* src, int64_t nbits);
+
+// ---- host staging of pipeline breakers (tg_agg_push / tg_sort_push) ------------------------------------------------
+// Child chunks arrive as small host chunks (1024 rows) with an optional sel vector; they are appended, sel applied, into
+// pinned buffers that are flushed to the device in batches of millions of rows.  Per column: 8-byte values and, once any
+// chunk carried a bitmap, a null bitmap (earlier rows all NOT NULL).  Only columns with needed[c] != 0 are staged.
+struct ColumnStage {
+  std::vector<std::unique_ptr<PinBuf>> data, nulls;
+  std::vector<char> has_nulls;
+  int64_t rows = 0;
+  void init(int ncols) {
+    for (int c = 0; c < ncols; c++) { data.emplace_back(new PinBuf()); nulls.emplace_back(new PinBuf()); }
+    has_nulls.assign(ncols, 0);
+  }
+};
+inline int64_t logical_rows(const tg_chunk* c) { return c->sel ? c->nsel : (c->ncols > 0 ? c->cols[0].length : 0); }
+int stage_append(ColumnStage& st, const tg_chunk* chk, const std::vector<char>& needed);
+
+// Copy rows [lo, lo + want) of ncols device-resident 8-byte columns to the caller's host chunk (the Next of a pipeline
+// breaker).  bitmaps[k] = packed device null bitmap of column k, or nullptr when the column has no NULLs.  Any `lo` is
+// served: a bitmap slice that starts inside a byte is fetched whole and shifted on the host.  Synchronises `st`.
+int copy_out_rows(cudaStream_t st, int ncols, const void* const* cols, const uint8_t* const* bitmaps, int64_t lo,
+                  int64_t want, tg_mut_chunk* out, int64_t* d2h_bytes);
 
 // device ordinal guard
 struct DeviceGuard {

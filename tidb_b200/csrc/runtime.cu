@@ -37,6 +37,72 @@ void append_bits(uint8_t* dst, int64_t pos, const uint8_t* src, int64_t nbits) {
   if (((pos + nbits + 7) >> 3) > d + nbytes) dst[d + nbytes] = carry;
 }
 
+int stage_append(ColumnStage& st, const tg_chunk* chk, const std::vector<char>& needed) {
+  int64_t n = logical_rows(chk);
+  if (n == 0) return TG_OK;
+  for (size_t c = 0; c < needed.size(); c++) {
+    if (!needed[c]) continue;
+    const tg_column& col = chk->cols[c];
+    PinBuf& d = *st.data[c];
+    TG_TRY(d.reserve((size_t)(st.rows + n) * 8));
+    uint64_t* dst = reinterpret_cast<uint64_t*>(d.p) + st.rows;
+    const uint64_t* src = reinterpret_cast<const uint64_t*>(col.data);
+    if (!chk->sel) std::memcpy(dst, src, (size_t)n * 8);
+    else for (int64_t i = 0; i < n; i++) dst[i] = src[chk->sel[i]];
+    d.used = (size_t)(st.rows + n) * 8;
+    bool bring = col.null_bitmap != nullptr;
+    if (bring || st.has_nulls[c]) {
+      PinBuf& nb = *st.nulls[c];
+      size_t need = (size_t)((st.rows + n + 7) / 8) + 1;
+      TG_TRY(nb.reserve(need));
+      if (!st.has_nulls[c]) { std::memset(nb.p, 0xff, (size_t)((st.rows + 7) / 8) + 1); st.has_nulls[c] = 1; }
+      if (bring && !chk->sel) append_bits(nb.p, st.rows, col.null_bitmap, n);
+      else for (int64_t i = 0; i < n; i++) {
+        bool nn = bring ? bit_not_null(col.null_bitmap, chk->sel ? chk->sel[i] : i) : true;
+        int64_t r = st.rows + i;
+        if (nn) nb.p[r >> 3] |= (uint8_t)(1u << (r & 7)); else nb.p[r >> 3] &= (uint8_t)~(1u << (r & 7));
+      }
+      nb.used = need;
+    }
+  }
+  st.rows += n;
+  return TG_OK;
+}
+
+int copy_out_rows(cudaStream_t st, int ncols, const void* const* cols, const uint8_t* const* bitmaps, int64_t lo,
+                  int64_t want, tg_mut_chunk* out, int64_t* d2h_bytes) {
+  const int shift = (int)(lo & 7);
+  std::vector<std::vector<uint8_t>> shifted;
+  for (int k = 0; k < ncols; k++) {
+    TG_CUDA(cudaMemcpyAsync(out->cols[k].data, reinterpret_cast<const uint8_t*>(cols[k]) + (size_t)lo * 8, (size_t)want * 8, cudaMemcpyDeviceToHost, st));
+    *d2h_bytes += want * 8;
+    size_t nb = (size_t)((want + 7) / 8);
+    if (bitmaps[k]) {
+      if (!out->cols[k].null_bitmap) return fail(TG_ERR_INVALID, "output column can be NULL but the caller passed no null bitmap");
+      if (shift == 0) TG_CUDA(cudaMemcpyAsync(out->cols[k].null_bitmap, bitmaps[k] + lo / 8, nb, cudaMemcpyDeviceToHost, st));
+      else {
+        shifted.emplace_back((size_t)((shift + want + 7) / 8) + 1, (uint8_t)0);
+        TG_CUDA(cudaMemcpyAsync(shifted.back().data(), bitmaps[k] + lo / 8, shifted.back().size() - 1, cudaMemcpyDeviceToHost, st));
+      }
+    } else if (out->cols[k].null_bitmap) {
+      std::memset(out->cols[k].null_bitmap, 0xff, nb);
+      if (want & 7) out->cols[k].null_bitmap[nb - 1] = (uint8_t)((1u << (want & 7)) - 1);
+    }
+  }
+  TG_CUDA(cudaStreamSynchronize(st));
+  if (shift) {
+    size_t q = 0;
+    for (int k = 0; k < ncols; k++) {
+      if (!bitmaps[k]) continue;
+      const std::vector<uint8_t>& src = shifted[q++];
+      size_t nb = (size_t)((want + 7) / 8);
+      for (size_t b = 0; b < nb; b++) out->cols[k].null_bitmap[b] = (uint8_t)((src[b] >> shift) | (src[b + 1] << (8 - shift)));
+    }
+  }
+  if (want & 7) for (int k = 0; k < ncols; k++) if (bitmaps[k]) out->cols[k].null_bitmap[want >> 3] &= (uint8_t)((1u << (want & 7)) - 1);
+  return TG_OK;
+}
+
 cudaStream_t service_stream(int device) {
   static std::mutex mu;
   static cudaStream_t streams[64];

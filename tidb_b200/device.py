@@ -1,6 +1,6 @@
 """Device-resident ("synthetic columnar") entry points: columns live in HBM as torch tensors, the
 operators run through the same C-ABI handles (tg_join_build_push_dev / tg_join_probe_dev /
-tg_agg_push_dev).  torch is plumbing here — device memory, streams, torch.distributed — never compute.
+tg_agg_push_dev / tg_sort_push_dev).  torch is plumbing here — device memory, streams, torch.distributed — never compute.
 """
 from __future__ import annotations
 
@@ -116,6 +116,49 @@ class DeviceAgg:
     def close(self) -> None:
         if self.h:
             self.lib.tg_agg_close(self.h)
+            self.h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class DeviceSort:
+    """One tg_sort handle driven with device-resident chunks (tg_sort_push_dev; the columns are borrowed until finish)."""
+
+    def __init__(self, schema, by_items, device: int = 0, expected_rows: int = 0, stream: Optional[int] = None):
+        self.lib = abi.load_lib()
+        desc, self._keep = abi.sort_desc(schema, by_items, device, expected_rows, stream)
+        self.h = C.c_void_p()
+        abi.check(self.lib.tg_sort_open(C.byref(desc), C.byref(self.h)))
+        self.n_out = len(schema)
+        self._pushed = []
+
+    def push(self, cols: Sequence[torch.Tensor], nulls=None) -> None:
+        ck = dev_chunk(cols, nulls)
+        abi.check(self.lib.tg_sort_push_dev(self.h, C.byref(ck)))
+        self._pushed.append(ck)
+
+    def finish(self) -> Tuple[int, List[int], List[int]]:
+        """-> (rows, device pointers of the sorted columns, of their null bitmaps or 0)"""
+        abi.check(self.lib.tg_sort_finish(self.h))
+        self._pushed = []
+        out_cols = (C.c_void_p * self.n_out)()
+        out_nulls = (C.c_void_p * self.n_out)()
+        rows = C.c_int64(0)
+        abi.check(self.lib.tg_sort_result_dev(self.h, C.byref(rows), out_cols, out_nulls))
+        return rows.value, [p or 0 for p in out_cols], [p or 0 for p in out_nulls]
+
+    def stats(self) -> abi.TgSortStats:
+        s = abi.TgSortStats()
+        abi.check(self.lib.tg_sort_get_stats(self.h, C.byref(s)))
+        return s
+
+    def close(self) -> None:
+        if self.h:
+            self.lib.tg_sort_close(self.h)
             self.h = C.c_void_p()
 
     def __del__(self):

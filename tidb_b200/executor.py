@@ -5,7 +5,8 @@ Open(ctx) / Next(ctx, req *chunk.Chunk) / Close(), children pulled with exec.Nex
 zero rows = EOF.  A cgo shim implementing that interface forwards to the C-ABI exactly like the
 classes below do (INTEGRATION.md shows the Go source); they exist in Python only because this image
 has no Go toolchain.  Names follow the reference: MockDataSource (internal/testutil/testutil.go:63),
-HashJoinV2Exec (join/hash_join_v2.go:608), HashAggExec (aggregate/agg_hash_executor.go:93).
+HashJoinV2Exec (join/hash_join_v2.go:608), HashAggExec (aggregate/agg_hash_executor.go:93), SortExec
+(sortexec/sort.go:43).
 
 There is no CPU fallback: every operator fails if libtidbgpu.so is missing or no CUDA device exists.
 """
@@ -410,6 +411,59 @@ class TopNExec(Executor):
         if hi <= lo:
             return self.empty_chunk()
         return Chunk([Column(c.data[lo:hi], c.nulls()[lo:hi] if c.nulls().any() else None) for c in self._result.columns])
+
+
+class SortExec(Executor):
+    """GPU replacement of sortexec.SortExec (pkg/executor/sortexec/sort.go:43) for ORDER BY without LIMIT: a pipeline
+    breaker.  Open opens a tg_sort handle (sort.go:155); the first Next pushes every child chunk, sel vectors included
+    (fetchChunks sort.go:526), and sorts on the device (tg_sort_finish); each Next then returns at most `required_rows`
+    rows of the child's schema in ORDER BY order (sort.go:265).  by_items = [(column, desc)], plain column references."""
+
+    def __init__(self, child: Executor, by_items: Sequence, device: int = 0):
+        super().__init__(child.schema, [child])
+        self.by_items, self.device = [(int(c), bool(d)) for c, d in by_items], device
+        self._h = C.c_void_p()
+        self._lib = None
+        self._prepared = False
+        self._out: Optional[MutChunk] = None
+
+    def open(self) -> None:
+        super().open()
+        self._lib = abi.load_lib()
+        desc, keep = abi.sort_desc(self.schema, self.by_items, self.device)
+        self._h = C.c_void_p()
+        abi.check(self._lib.tg_sort_open(C.byref(desc), C.byref(self._h)))
+        self._prepared = False
+
+    def next(self, required_rows: int = MAX_CHUNK_SIZE) -> Chunk:
+        if not self._h:
+            raise RuntimeError("next before open")
+        if not self._prepared:
+            while True:
+                chk = self.children[0].next(MAX_CHUNK_SIZE)
+                if chk.num_rows() == 0:
+                    break
+                cs = chk.to_struct()
+                abi.check(self._lib.tg_sort_push(self._h, C.byref(cs)))
+            abi.check(self._lib.tg_sort_finish(self._h))
+            self._prepared = True
+        if self._out is None or self._out.capacity < required_rows:
+            self._out = _out_chunk(self.schema, max(required_rows, 8))
+        n = C.c_int64(0)
+        abi.check(self._lib.tg_sort_next(self._h, C.byref(self._out.struct), C.c_int64(required_rows), C.byref(n)))
+        cols = self._out.columns(n.value)
+        return Chunk([Column(v, nl if nl.any() else None) for v, nl in cols])
+
+    def stats(self) -> abi.TgSortStats:
+        s = abi.TgSortStats()
+        abi.check(self._lib.tg_sort_get_stats(self._h, C.byref(s)))
+        return s
+
+    def close(self) -> None:
+        if self._h:
+            self._lib.tg_sort_close(self._h)
+            self._h = C.c_void_p()
+        super().close()
 
 
 def drain(e: Executor, required_rows: int = MAX_CHUNK_SIZE) -> List[Chunk]:
